@@ -77,7 +77,11 @@ def parse_args():
     ap.add_argument("--stats", action="store_true", help="RG_CFG_STATS: event counters of k_eval_or_ms in the line")
     ap.add_argument("--maxscore", action="store_true",
                     help="RG_CFG_MAXSCORE: disjunctions through k_eval_or_ms (bitmaps + per-document bound) (A/B runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the TopDocs of the last timed step of the headline workload to DIR/*.npy")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     w = dict(WORKLOADS[a.workload])
     for key in ("docs", "terms", "batch", "k"):
         if getattr(a, key):
@@ -405,13 +409,11 @@ def run_workload(ctx, name, w, args, steps, warmup, cpu_queries, cpu_seconds, fl
         local_rec = torch.as_tensor(_CudaArray(rec_ptr, per_rank * rec_bytes * nq), device=dev)
         gathered = torch.empty(world * per_rank * rec_bytes * nq, dtype=torch.uint8, device=dev)
 
-    def one_step(fetch=False):
+    def one_step():
         batch.run()
-        if world > 1:  # kernels -> one all-gather -> leaf-order merge, all on one stream; the copy back only on request
+        if world > 1:  # kernels -> one all-gather -> leaf-order merge, all on one stream; the result stays on the device
             dist.all_gather_into_tensor(gathered, local_rec)
             eng.merge_leaf_records_device(gathered.data_ptr(), n_seg, nq, k)
-            return eng.merge_fetch() if fetch else None
-        return batch.fetch() if fetch else None
 
     for _ in range(warmup):
         one_step()
@@ -432,7 +434,8 @@ def run_workload(ctx, name, w, args, steps, warmup, cpu_queries, cpu_seconds, fl
         dist.all_reduce(ms_total, op=dist.ReduceOp.MAX)
     ms_step = float(ms_total[0]) / steps
     launches = eng.launch_count() - launches0
-    result = one_step(fetch=True)
+    # the TopDocs of the last timed step, copied back without running the batch again
+    result = batch.fetch() if world == 1 else eng.merge_fetch()
     if world > 1:
         batch.fetch()  # populates the per-kernel CUDA-event timings of the last run
     eval_ms = eng.last_kernel_ms("eval")
@@ -469,7 +472,7 @@ def run_workload(ctx, name, w, args, steps, warmup, cpu_queries, cpu_seconds, fl
         b2.close()
         return res
 
-    e2e_steps = max(1, min(steps, 3))
+    e2e_steps = steps
     fresh = [build_query_arrays(gen_queries(name, w["terms"], w["batch"], w["seed_queries"] + 7919 * (i + 1)), weight_of, engine)
              for i in range(e2e_steps)]
     e2e_res = e2e_step(q, c)
@@ -609,7 +612,7 @@ def run_workload(ctx, name, w, args, steps, warmup, cpu_queries, cpu_seconds, fl
                                     "postings_per_s": float(costs[pick].sum() / dt)}
         out["cpu_baseline"] = cpu
         del ix
-    ctx.last_engine, ctx.last_batch = eng, batch
+    ctx.last_engine, ctx.last_batch, ctx.last_result = eng, batch, result
     return out
 
 
@@ -677,6 +680,31 @@ def decode_bench(eng, stream, have_full_index):
     return res
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, result):
+    """TopDocs as a caller of the timed path receives them, one row per query: doc ids (float64: exact for every
+    int32), scores (float32), hit counts and total hits.  Slots past a row's hit count are not part of its TopDocs
+    and are written as doc -1, score 0.  Above DUMP_LIMIT_BYTES a fixed seeded sample of rows is written;
+    query_rows.npy holds the batch index of each row."""
+    hits, counts, total = result
+    nq, k = hits.shape
+    rows = np.arange(nq)
+    row_bytes = k * (8 + 4) + 8 + 8 + 8
+    if nq * row_bytes > DUMP_LIMIT_BYTES:
+        rows = np.sort(np.random.default_rng(0x5EED00D0).choice(nq, DUMP_LIMIT_BYTES // row_bytes, replace=False))
+    hits, counts, total = hits[rows], counts[rows], total[rows]
+    valid = np.arange(k)[None, :] < counts[:, None]
+    arrays = {"docs": np.where(valid, hits["doc"], -1).astype(np.float64),
+              "scores": np.where(valid, hits["score"], np.float32(0)).astype(np.float32),
+              "counts": counts.astype(np.float64), "total_hits": total.astype(np.float64),
+              "query_rows": rows.astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def load_traffic():
     try:
         with open(os.path.join(ROOT, "profiles", "r2_traffic.json")) as f:
@@ -718,6 +746,8 @@ def main():
     name, w = args.workload, args.w
     main_res = run_workload(ctx, name, w, args, args.steps, args.warmup, args.cpu_sample, args.cpu_seconds, flags=flags)
     eng, batch = ctx.last_engine, ctx.last_batch
+    if args.dump_outputs and ctx.rank == 0:
+        dump_outputs(args.dump_outputs, ctx.last_result)
     decode = None
     if ctx.rank == 0 and not args.no_decode:
         decode = decode_bench(eng, ctx.stream, have_full_index=True)
@@ -731,11 +761,11 @@ def main():
                           ("score_columns_no_scored_lists", engine.CFG_NO_LISTS),
                           ("bitmaps_per_document_bound", engine.CFG_MAXSCORE),
                           ("bitmaps_bound_with_tf_planes", engine.CFG_MAXSCORE | engine.CFG_TFPLANES)):
-            r = run_workload(ctx, name, w, args, 2, 1, 0, 0, flags=fl, light=True)
+            r = run_workload(ctx, name, w, args, args.steps, args.warmup, 0, 0, flags=fl, light=True)
             ab[label] = {"queries_per_s": r["value"], "ms_per_step": r["ms_per_step"]}
         if ctx.world == 1:
             for other in ("c3", "c5"):
-                r = run_workload(ctx, other, dict(WORKLOADS[other]), args, max(3, args.steps), 3, 256, 8.0)
+                r = run_workload(ctx, other, dict(WORKLOADS[other]), args, args.steps, args.warmup, 256, 8.0)
                 ctx.last_batch.close()
                 ctx.last_engine.close()
                 extra[other] = {kk: r[kk] for kk in ("value", "ms_per_step", "config", "e2e", "first_batch_ms", "roofline",
